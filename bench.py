@@ -6,6 +6,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference --steps K --warmup W      # CPU arm (oracle port of the reference)
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR   # also write the last timed step's outputs
 
 A "step" is one forward pass over one synthetic batch (the hot path named by BASELINE.json's
 north_star; the reference publishes no throughput, so vs_baseline is null). Rank 0 prints ONE JSON
@@ -113,6 +114,22 @@ class ClockSampler:
                     reasons.add(n)
         return {"sm_mhz": statistics.median(sm) if sm else None, "sm_max_mhz": max(smax) if smax else None,
                 "samples": len(sm), "reasons": sorted(reasons)}
+
+
+def dump_outputs(path, outs, limit=64 * 10**6):
+    """Writes every output tensor as <path>/<name>.npy in float32 (rank 0's last timed step). When they exceed `limit`
+    bytes in all, each is cut to the same fraction of its elements, at flat indices drawn (sorted) from a generator with
+    a fixed seed, so two runs of the same command write the same positions."""
+    import numpy as np
+
+    os.makedirs(path, exist_ok=True)
+    host = {k: v.detach().float().cpu() for k, v in outs.items()}
+    keep = min(1.0, (limit - 4096 * len(host)) / (4 * sum(v.numel() for v in host.values())))
+    for k, v in host.items():
+        if keep < 1.0:
+            idx = torch.randperm(v.numel(), generator=torch.Generator().manual_seed(0))[:int(v.numel() * keep)]
+            v = v.reshape(-1)[idx.sort().values]
+        np.save(os.path.join(path, f"{k}.npy"), v.numpy())
 
 
 # ------------------------------------------------------------------------------------------------
@@ -354,6 +371,15 @@ def run_ours(args):
     launches_per_fwd = plan.launches_per_forward()
     torch.cuda.synchronize()
 
+    def flat(o):      # InvPT returns {'task': ..., 'inter_preds': {'task': ...}}: every tensor is read back
+        r = {}
+        for k, v in o.items():
+            if isinstance(v, dict):
+                r.update({f"{k}.{k2}": v2 for k2, v2 in v.items()})
+            else:
+                r[k] = v
+        return r
+
     # ---------------- device-resident throughput ("value")
     with torch.no_grad():
         for i in range(args.warmup):
@@ -372,24 +398,19 @@ def run_ours(args):
         s.record()
         with torch.no_grad():
             for i in range(args.steps):
-                model(dev_in[i % n_rot])
+                last = model(dev_in[i % n_rot])
         e.record()
         torch.cuda.synchronize()
         barrier(world)
         regions.append(max_over_ranks(s.elapsed_time(e), world, dev))
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, flat(last))   # before the next call reuses the output buffers
+    del last
     ms_total = sorted(regions)[len(regions) // 2]
     value = world * B * args.steps / (ms_total * 1e-3)
 
     # ---------------- end to end through the public call, host buffers, H2D + D2H inside the timed region
-    def flat(o):      # InvPT returns {'task': ..., 'inter_preds': {'task': ...}}: every tensor is read back
-        r = {}
-        for k, v in o.items():
-            if isinstance(v, dict):
-                r.update({f"{k}.{k2}": v2 for k2, v2 in v.items()})
-            else:
-                r[k] = v
-        return r
     out = flat(out)
     out_bytes = sum(v.numel() * v.element_size() for v in out.values())
     in_bytes = host_in[0].numel() * 4
@@ -602,7 +623,7 @@ def train_eager_baseline(cfg_name, batch, dev, labels, steps=3, warmup=1):
     return res
 
 
-def train_leg(args, rank, world, dev, steps=10, warmup=3, repeats=3):
+def train_leg(args, rank, world, dev, warmup=3, repeats=3):
     """The TRAINING step of the same workload on the same ranks, appended to the inference line as `train_step`: the
     forward shards over the batch without any exchange, so the scaling run would otherwise never exercise a collective.
     Here every step all-reduces the SyncBatchNorm statistics and the whole gradient arena over NCCL (captured with the
@@ -611,6 +632,7 @@ def train_leg(args, rank, world, dev, steps=10, warmup=3, repeats=3):
     from mtt_b200 import dist as D
     from mtt_b200.train import TrainStep
 
+    steps = args.steps
     cfg, M, _ = family(args.config)
     nsplit = 2 if args.mode == "parity" else 1
     torch.manual_seed(0)
@@ -868,7 +890,7 @@ def run_reference_train(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps per timed region")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--mode", default="parity", choices=["parity", "speed"])
@@ -883,7 +905,13 @@ def main():
                     help="skip the `train_step` block (the training step timed on the same ranks after the forward)")
     ap.add_argument("--train-leg-timeout", type=float, default=150.0,
                     help="seconds after which the watchdog prints the finished inference line without the train_step block")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="forward benchmark: write the outputs of the last timed step as DIR/<name>.npy (float32, <= 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.train or args.impl != "ours"):
+        ap.error("--dump-outputs covers the forward benchmark (--impl ours without --train)")
     if args.config not in WORKLOAD:       # any named configuration of mtt_b200/configs.py (tiny ones: contract tests)
         try:
             family(args.config)

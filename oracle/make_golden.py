@@ -351,6 +351,150 @@ def main_train(only=None):
         print(f"wrote {path} ({os.path.getsize(path) / 1024:.0f} KiB)", flush=True)
 
 
+# ---------------------------------------------------------------------------------------------------------
+# Reference checks (tests/golden/reference_checks.pt): the reference's outputs for the comparisons of
+# tests/test_oracle.py and tests/test_random_configs.py, so those tests run where the reference is absent.
+# Weights are the oracle initialisers plus the perturbations `perturb` draws from a fixed CPU generator
+# (BatchNorm statistics; Swin also bias tables and biases), loaded into the reference with strict=True; the
+# fixture stores a summary of each output (`summarize`) and signatures of the reference's parameter names.
+SAMPLE_STRIDE = 1000003        # prime: the sampled flat indices are distinct for any output smaller than it
+
+
+def signature(pairs):
+    """SHA-256 over a sequence of (name, shape) pairs, in the order given."""
+    h = hashlib.sha256()
+    for k, shape in pairs:
+        h.update(f"{k}:{tuple(shape)};".encode())
+    return h.hexdigest()
+
+
+def perturb(sd, seed, swin=False):
+    """A copy of state dict `sd` (same order) with BatchNorm running statistics drawn around (0, 1); with `swin`, also
+    relative-position bias tables ~ N(0, 0.5) and every bias ~ N(0, 0.05)."""
+    g = torch.Generator().manual_seed(seed)
+    out = {}
+    for k, v in sd.items():
+        if k.endswith("running_mean"):
+            v = torch.randn(v.shape, generator=g) * 0.1
+        elif k.endswith("running_var"):
+            v = torch.rand(v.shape, generator=g) * 0.4 + 0.8
+        elif swin and "relative_position_bias_table" in k:
+            v = torch.randn(v.shape, generator=g) * 0.5
+        elif swin and k.endswith(".bias"):
+            v = torch.randn(v.shape, generator=g) * 0.05
+        out[k] = v
+    return out
+
+
+def summarize(y, k=256):
+    """Output tensor [B, C, ...] -> k elements at fixed flat indices, the per-(image, channel) means (float64), the norm."""
+    y = y.detach().float().cpu()
+    n = y.numel()
+    assert n % SAMPLE_STRIDE, n
+    idx = (torch.arange(min(k, n), dtype=torch.int64) * SAMPLE_STRIDE + 7) % n
+    return {"shape": tuple(y.shape), "sample": y.reshape(-1)[idx].clone(),
+            "channel_mean": y.double().flatten(2).mean(2), "norm": float(y.double().norm()), "absmax": float(y.abs().max())}
+
+
+def max_abs_error(y, rec):
+    """Largest |difference| of y against a `summarize` record, over the sampled elements and the channel means (each a
+    lower bound of the largest elementwise |difference|)."""
+    s = summarize(y)
+    assert s["shape"] == rec["shape"], (s["shape"], rec["shape"])
+    return max(float((s["sample"] - rec["sample"]).abs().max()), float((s["channel_mean"] - rec["channel_mean"]).abs().max()))
+
+
+def rel_l2_error(y, rec):
+    """Relative L2 difference of y against a `summarize` record: over the sampled elements, and | |y| - |ref| | / |ref|
+    (a lower bound of |y - ref| / |ref|)."""
+    s = summarize(y)
+    assert s["shape"] == rec["shape"], (s["shape"], rec["shape"])
+    return max(float((s["sample"] - rec["sample"]).norm() / rec["sample"].norm()), abs(s["norm"] - rec["norm"]) / rec["norm"])
+
+
+# named configurations of tests/test_oracle.py: (family, config, seed, batch)
+REF_NAMED = [("tp", "tp_tiny", 101, 2), ("tp", "tp_tiny1", 102, 2), ("tp", "tp_tiny_de", 103, 2), ("ip", "ip_tiny", 104, 2),
+             ("ip", "ip_cfg1", 105, 2), ("tps", "tps_tiny", 106, 2), ("tps", "tps_tiny4", 107, 2), ("tps", "tps_mid", 108, 1)]
+SELECT_LISTS = [[1, 2, 4], [0, 2, 3], [2, 2, 3], [3, 2, 1]]
+
+
+def _reference_run(fam, cfg, sd, x):
+    build = {"tp": ref_loader.build_taskprompter, "ip": ref_loader.build_invpt, "tps": ref_loader.build_taskprompter_swin}[fam]
+    model = build(cfg).eval()
+    ref_sd = model.state_dict()
+    if fam == "tps":
+        missing, unexpected = model.load_state_dict(sd, strict=False)   # index / mask buffers are derived, not stored
+        assert not unexpected and all("relative_position_index" in k or "attn_mask" in k for k in missing)
+    else:
+        model.load_state_dict(sd, strict=True)
+    with torch.no_grad():
+        y = model(x)
+    rec = {"out": {t: summarize(y[t]) for t in cfg["tasks"]},
+           "inter_preds": {t: summarize(y["inter_preds"][t]) for t in cfg["tasks"]} if fam == "ip" else None}
+    derived = ("relative_position_index", "attn_mask")
+    params = [(k, v.shape) for k, v in ref_sd.items() if not any(d in k for d in derived)]
+    return rec, params
+
+
+def _reference_raises(fam, cfg, x):
+    build = ref_loader.build_invpt if fam == "ip" else ref_loader.build_taskprompter_swin
+    try:
+        with torch.no_grad():
+            build(cfg).eval()(x)
+    except (RuntimeError, AssertionError) as ex:
+        return type(ex).__name__
+    return None
+
+
+def make_reference_checks():
+    import importlib
+
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    import test_random_configs as RC
+
+    oracle_of = {"tp": "oracle.taskprompter_ref", "ip": "oracle.invpt_ref", "tps": "oracle.taskprompter_swin_ref"}
+    cases = {}
+    for fam, name, seed, batch in REF_NAMED:
+        cfg = (configs.taskprompter if fam == "tp" else configs.invpt if fam == "ip" else configs.taskprompter_swin)(name)
+        sd = perturb(importlib.import_module(oracle_of[fam]).init_state_dict(cfg, seed=seed), seed + 1, swin=fam == "tps")
+        x = torch.randn(batch, 3, *cfg["img_size"], generator=torch.Generator().manual_seed(seed + 1000))
+        rec, params = _reference_run(fam, cfg, sd, x)
+        rec.update(seed=seed, batch=batch, sorted_param_signature=signature(sorted(params)))
+        cases[name] = rec
+    for seed in range(6):                   # test_oracle_vs_reference_on_random_geometries
+        cfg, B = RC.draw(seed)
+        sd = perturb(importlib.import_module(oracle_of["tp"]).init_state_dict(cfg, seed=seed), seed + 1)
+        x = torch.randn(B, 3, *cfg["img_size"], generator=torch.Generator().manual_seed(seed + 1000))
+        cases[f"random_tp{seed}"] = _reference_run("tp", cfg, sd, x)[0]
+    for seed in range(6):                   # test_invpt_launch_plan_and_oracle_on_random_geometries: the test's own weights
+        cfg, B = RC.draw_invpt(seed)
+        torch.manual_seed(seed)
+        x = torch.randn(B, 3, *cfg["img_size"])
+        cases[f"random_ip{seed}"] = _reference_run("ip", cfg, importlib.import_module(oracle_of["ip"]).init_state_dict(cfg, seed=seed), x)[0]
+    for seed in range(8):                   # test_swin_launch_plan_and_oracle_on_random_geometries: the test's own weights
+        cfg, B = RC.draw_swin(seed)
+        torch.manual_seed(seed)
+        x = torch.randn(B, 3, *cfg["img_size"])
+        sd = importlib.import_module(oracle_of["tps"]).init_state_dict(cfg, seed=seed)
+        cases[f"random_swin{seed}"] = _reference_run("tps", cfg, sd, x)[0]
+    for sel in SELECT_LISTS:                # test_unusual_select_lists_follow_the_reference
+        cfg = dict(RC._TP_BASE, select=sel)
+        sd = perturb(importlib.import_module(oracle_of["tp"]).init_state_dict(cfg, seed=5), 6)
+        x = torch.randn(2, 3, 64, 64, generator=torch.Generator().manual_seed(1005))
+        cases["select_" + "-".join(map(str, sel))] = _reference_run("tp", cfg, sd, x)[0]
+    raises = {"ip_6x6": _reference_raises("ip", dict(tasks=["edge", "semseg"], num_output={"edge": 1, "semseg": 5},
+                                                     img_size=(96, 96), patch=16, C=128, depth=4, heads=2, select=[1, 2, 3],
+                                                     embed_dim=32, pred_const=16, down=2, name="ip_6x6"), torch.randn(1, 3, 96, 96))}
+    for change, match in RC.SWIN_REJECTS:
+        cfg = dict(RC.SWIN_BAD, **change)
+        raises[match] = _reference_raises("tps", cfg, torch.randn(1, 3, *cfg["img_size"]))
+    swin_b = ref_loader.build_taskprompter_swin(configs.taskprompter_swin("tps_swinB")).state_dict()
+    params = sorted((k, v.shape) for k, v in swin_b.items() if "relative_position_index" not in k and "attn_mask" not in k)
+    return {"family": "reference_checks", "cases": cases, "raises": raises,
+            "tps_swinB": {"sorted_param_signature": signature(params), "n_params": len(params)}, "torch": torch.__version__,
+            "made_by": "oracle/make_golden.py refchecks: the unmodified reference forward (eval, fp32, CPU), summarised"}
+
+
 def main():
     if not ref_loader.available():
         raise SystemExit("reference not found (set MTT_REFERENCE or mount /root/reference)")
@@ -389,5 +533,11 @@ if __name__ == "__main__":
         if not ref_loader.available():
             raise SystemExit("reference not found (set MTT_REFERENCE or mount /root/reference)")
         main_train(set(sys.argv[2:]) or None)
+    elif len(sys.argv) > 1 and sys.argv[1] == "refchecks":   # python -m oracle.make_golden refchecks
+        if not ref_loader.available():
+            raise SystemExit("reference not found (set MTT_REFERENCE to the reference tree)")
+        path = os.path.join(GOLD, "reference_checks.pt")
+        torch.save(make_reference_checks(), path)
+        print(f"wrote {path} ({os.path.getsize(path) / 1024:.0f} KiB)")
     else:
         main()

@@ -1,5 +1,8 @@
-"""CPU: the oracle restatement against (a) the golden vectors produced by the unmodified reference and
-(b) the reference itself when /root/reference is present (build container)."""
+"""CPU: the oracle restatement against the golden vectors produced by the unmodified reference: (a) with the oracle's
+initialisers (tests/golden/<config>.pt) and (b) with perturbed BatchNorm statistics (Swin: also bias tables and biases),
+checked against summaries of the reference's outputs and signatures of its parameter names
+(tests/golden/reference_checks.pt, `python -m oracle.make_golden refchecks`). The state-dict sharing of accelerate()
+needs a live instance of the reference's classes and runs where the reference tree is present."""
 import os
 
 import pytest
@@ -8,9 +11,13 @@ import torch
 from oracle import configs, ref_loader
 from oracle import taskprompter_ref as TPR
 from oracle import invpt_ref as IPR
-from oracle.make_golden import sd_checksum
+from oracle.make_golden import max_abs_error, perturb, sd_checksum, signature
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+
+
+def reference_case(name):
+    return torch.load(os.path.join(GOLD, "reference_checks.pt"), weights_only=False)["cases"][name]
 
 
 @pytest.mark.parametrize("name", ["tp_tiny", "tp_tiny1", "tp_tiny_de"])
@@ -28,22 +35,17 @@ def test_taskprompter_oracle_vs_golden(name):
             assert torch.equal(out[t].argmax(1), ref.argmax(1))
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="reference tree not present")
 @pytest.mark.parametrize("name", ["tp_tiny", "tp_tiny1", "tp_tiny_de"])
 def test_taskprompter_oracle_vs_reference(name):
+    rec = reference_case(name)
     cfg = configs.taskprompter(name)
-    torch.manual_seed(0)
-    model = ref_loader.build_taskprompter(cfg).eval()     # the reference's own initialisation
-    for m in model.modules():
-        if isinstance(m, torch.nn.BatchNorm2d):
-            m.running_mean.normal_(0, 0.1)
-            m.running_var.uniform_(0.8, 1.2)
-    x = torch.randn(2, 3, *cfg["img_size"])
+    sd = perturb(TPR.init_state_dict(cfg, seed=rec["seed"]), rec["seed"] + 1)
+    assert signature(sorted((k, v.shape) for k, v in sd.items())) == rec["sorted_param_signature"]   # the reference's names
+    x = torch.randn(rec["batch"], 3, *cfg["img_size"], generator=torch.Generator().manual_seed(rec["seed"] + 1000))
     with torch.no_grad():
-        ref = model(x)
-        out = TPR.forward(model.state_dict(), cfg, x)
+        out = TPR.forward(sd, cfg, x)
     for t in cfg["tasks"]:
-        assert (out[t] - ref[t]).abs().max() <= 2e-6, t
+        assert max_abs_error(out[t], rec["out"][t]) <= 2e-6, t
 
 
 @pytest.mark.skipif(not ref_loader.available(), reason="reference tree not present")
@@ -74,23 +76,18 @@ def test_invpt_oracle_vs_golden(name):
             assert (out["inter_preds"][t] - fx["inter_preds"][t]).abs().max() <= 5e-6, t
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="reference tree not present")
 @pytest.mark.parametrize("name", ["ip_tiny", "ip_cfg1"])
 def test_invpt_oracle_vs_reference(name):
+    rec = reference_case(name)
     cfg = configs.invpt(name)
-    torch.manual_seed(0)
-    model = ref_loader.build_invpt(cfg).eval()
-    for m in model.modules():
-        if isinstance(m, (torch.nn.BatchNorm2d, torch.nn.SyncBatchNorm)):
-            m.running_mean.normal_(0, 0.1)
-            m.running_var.uniform_(0.8, 1.2)
-    x = torch.randn(2, 3, *cfg["img_size"])
+    sd = perturb(IPR.init_state_dict(cfg, seed=rec["seed"]), rec["seed"] + 1)
+    assert signature(sorted((k, v.shape) for k, v in sd.items())) == rec["sorted_param_signature"]
+    x = torch.randn(rec["batch"], 3, *cfg["img_size"], generator=torch.Generator().manual_seed(rec["seed"] + 1000))
     with torch.no_grad():
-        ref = model(x)
-        out = IPR.forward(model.state_dict(), cfg, x)
+        out = IPR.forward(sd, cfg, x)
     for t in cfg["tasks"]:
-        assert (out[t] - ref[t]).abs().max() <= 5e-6, t
-        assert (out["inter_preds"][t] - ref["inter_preds"][t]).abs().max() <= 5e-6, t
+        assert max_abs_error(out[t], rec["out"][t]) <= 5e-6, t
+        assert max_abs_error(out["inter_preds"][t], rec["inter_preds"][t]) <= 5e-6, t
 
 
 @pytest.mark.skipif(not ref_loader.available(), reason="reference tree not present")
@@ -124,38 +121,22 @@ def test_swin_oracle_vs_golden(name):
             assert torch.equal(out[t].argmax(1), ref.argmax(1))
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="reference tree not present")
 @pytest.mark.parametrize("name", ["tps_tiny", "tps_tiny4", "tps_mid"])
 def test_swin_oracle_vs_reference(name):
-    """Against the unmodified reference with ITS OWN initialisation (plus non-trivial biases, bias tables and
-    BatchNorm statistics): shifted and padded windows, 2x2 channel windows, patch merging of the logit maps."""
+    """Against the unmodified reference's outputs with non-trivial biases, bias tables and BatchNorm statistics: shifted
+    and padded windows, 2x2 channel windows, patch merging of the logit maps. The parameter names and shapes the oracle
+    expects are the reference module's (signature of the sorted list, derived index / mask buffers excluded)."""
     from oracle import taskprompter_swin_ref as SR
 
+    rec = reference_case(name)
     cfg = configs.taskprompter_swin(name)
-    torch.manual_seed(0)
-    model = ref_loader.build_taskprompter_swin(cfg).eval()
+    assert signature(sorted(SR.param_shapes(cfg).items())) == rec["sorted_param_signature"]
+    sd = perturb(SR.init_state_dict(cfg, seed=rec["seed"]), rec["seed"] + 1, swin=True)
+    x = torch.randn(rec["batch"], 3, *cfg["img_size"], generator=torch.Generator().manual_seed(rec["seed"] + 1000))
     with torch.no_grad():
-        for m in model.modules():
-            if isinstance(m, (torch.nn.BatchNorm2d, torch.nn.SyncBatchNorm)):
-                m.running_mean.normal_(0, 0.1)
-                m.running_var.uniform_(0.8, 1.2)
-        for k, v in model.named_parameters():
-            if "relative_position_bias_table" in k:
-                v.normal_(0, 0.5)
-            elif k.endswith(".bias"):
-                v.normal_(0, 0.05)
-    ref_sd = model.state_dict()
-    derived = {k for k in ref_sd if "relative_position_index" in k or "attn_mask" in k}
-    shapes = SR.param_shapes(cfg)
-    assert set(shapes) == set(ref_sd) - derived
-    assert all(tuple(ref_sd[k].shape) == tuple(shapes[k]) for k in shapes)
-    x = torch.randn(1 if name == "tps_mid" else 2, 3, *cfg["img_size"])
-    with torch.no_grad():
-        ref = model(x)
-        out = SR.forward(ref_sd, cfg, x)
+        out = SR.forward(sd, cfg, x)
     for t in cfg["tasks"]:
-        assert out[t].shape == ref[t].shape
-        assert (out[t] - ref[t]).abs().max() <= 5e-6, t
+        assert max_abs_error(out[t], rec["out"][t]) <= 5e-6, t
 
 
 def test_swin_window_tables_match_definitions():
@@ -171,18 +152,16 @@ def test_swin_window_tables_match_definitions():
     assert (m[3] != 0).any() and torch.equal(m[3], m[3].t())
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="reference tree not present")
 def test_swin_param_shapes_at_the_reference_config():
     """The reference's Cityscapes-3D Swin-B model (cs_swinB_taskprompter.yml: 1024x2048, img_ds_ratio 0.75, window 12,
     depths 2-2-18-2): every parameter name and shape the oracle expects equals the reference module's (274.6 M
-    parameters; construction only, no forward)."""
+    parameters; construction only, no forward; the reference's list is stored as a signature)."""
     from oracle import taskprompter_swin_ref as SR
 
     cfg = configs.taskprompter_swin("tps_swinB")
-    ref_sd = ref_loader.build_taskprompter_swin(cfg).state_dict()
-    derived = {k for k in ref_sd if "relative_position_index" in k or "attn_mask" in k}
+    ref = torch.load(os.path.join(GOLD, "reference_checks.pt"), weights_only=False)["tps_swinB"]
     shapes = SR.param_shapes(cfg)
-    assert set(shapes) == set(ref_sd) - derived and len(shapes) == 732
-    assert all(tuple(ref_sd[k].shape) == tuple(shapes[k]) for k in shapes)
+    assert len(shapes) == ref["n_params"] == 732
+    assert signature(sorted(shapes.items())) == ref["sorted_param_signature"]
     assert [SR.stage_geometry(cfg, i)[1] for i in range(4)] == [(192, 384), (96, 192), (48, 96), (24, 48)]
     assert [SR.level_resolution(cfg, i) for i in range(4)] == [(96, 192), (48, 96), (24, 48), (24, 48)]
